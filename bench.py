@@ -14,7 +14,7 @@ A "step" is one pass of ViDAR's two hot paths over one synthetic sample
        dvxlr autograd layer (`DifferentiableVoxelRendering`) forward + backward on them.
 metric = rays/sec = 30000 rays / step time (whole job); ms_per_step is the same thing as time.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 For N>1 launch under torchrun (one rank per GPU); the (camera, query) rows and the rays are
 sharded over ranks (strong scaling: total work fixed); per step one all-reduce of the BEV grid
 (the local scatter-add of SpatialCrossAttention's rows, 41 MB) and one of each grad_sigma.
@@ -277,10 +277,12 @@ def run_ours(args, light=False):
             # row-sharded in / out (the module's consumers in the encoder -- LayerNorm, FFN -- are row-wise): only the
             # 2.56 MB occupancy / feature / prob maps cross NVLink, never the 41 MB grid
             emb = embed.view(-1, EMBED)[lr0:lr1].detach().requires_grad_(True)
-            latent.forward_rows(emb, 1, GRID[1], GRID[2]).backward(grad_embed.view(-1, EMBED)[lr0:lr1])
+            lat = latent.forward_rows(emb, 1, GRID[1], GRID[2])
+            lat.backward(grad_embed.view(-1, EMBED)[lr0:lr1])
         else:
             emb = embed.detach().requires_grad_(True)
-            latent(emb).backward(grad_embed)
+            lat = latent(emb)
+            lat.backward(grad_embed)
         if record:
             e[3].record()
         sg = sigma[0].detach().requires_grad_(True)
@@ -304,7 +306,9 @@ def run_ours(args, light=False):
         if record:
             e[5].record()
             marks.append(e)
-        return bev.detach(), leaves, pred, grad_sigma, emb.grad, ce_grad, dv_grad
+        forward = dict(latent_out=lat.detach(), ray_ce_loss=ce.detach(), ray_ce_valid=valid, render_gt=gt,
+                       dvxlr_pred=dpred.detach())
+        return bev.detach(), leaves, pred, grad_sigma, emb.grad, ce_grad, dv_grad, forward
 
     def sync():
         torch.cuda.synchronize()
@@ -363,6 +367,10 @@ def run_ours(args, light=False):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         total_ms = float(t.item())
     ms_step = total_ms / args.steps
+    if getattr(args, "dump_outputs", None):
+        # `last` holds the last timed step: the captured graph's output buffers after its final replay, or the
+        # tensors of the last eager step
+        dump_outputs(args.dump_outputs, step_outputs(last))
     if graph is not None:
         # per-stage breakdown (and the roofline's kernel time): the same step launched eagerly with events between
         # the stages -- identical kernels, outside the headline's timed region
@@ -542,6 +550,39 @@ def run_ours(args, light=False):
     _finish(world)
 
 
+DUMP_SAMPLE = 1 << 20        # elements kept of a larger output: the 14 outputs of a step stay under 64 MB
+
+
+def step_outputs(last):
+    """{name: tensor} of what one step hands its caller: the forward results and the input gradients of every stage."""
+    bev, leaves, pred, grad_sigma, gemb, ce_grad, dv_grad, forward = last
+    out = {"msda_bev": bev}
+    for i, name in enumerate(("value", "sampling_loc", "attention_weights")):
+        out[f"msda_grad_{name}"] = torch.cat([t[i].grad.reshape(-1) for t in leaves])
+    out.update(latent_out=forward["latent_out"], latent_grad_embed=gemb, ray_ce_loss=forward["ray_ce_loss"],
+               ray_ce_valid=forward["ray_ce_valid"], ray_ce_grad_sigma=ce_grad, render_pred=pred,
+               render_gt=forward["render_gt"], render_grad_sigma=grad_sigma, dvxlr_pred=forward["dvxlr_pred"],
+               dvxlr_grad_sigma=dv_grad)
+    return out
+
+
+def dump_outputs(out_dir, arrays):
+    """Write every tensor as out_dir/<name>.npy in float32.  An output of more than DUMP_SAMPLE elements is
+    flattened and reduced to DUMP_SAMPLE of its elements, at ascending flat indices drawn from a fixed seed: the
+    same elements on every run, so two builds can be compared output for output."""
+    os.makedirs(out_dir, exist_ok=True)
+    total = 0
+    for name, t in arrays.items():
+        t = t.detach().float()
+        if t.numel() > DUMP_SAMPLE:
+            idx = np.sort(np.random.default_rng(0).choice(t.numel(), DUMP_SAMPLE, replace=False))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        a = t.cpu().numpy()
+        total += a.nbytes
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    assert total <= 64 << 20, f"--dump-outputs wrote {total} bytes"
+
+
 def check_sharded(dev, rank, world, grp, last, groups, msda_stage, grad_bev, latent, embed, grad_embed, sigma, origin,
                   rays_np, shapes, lsi, cam_groups):
     """Sharded == single GPU, checked on the lease the scaling run gets (SCALE_rNN.json carries the result).
@@ -551,7 +592,7 @@ def check_sharded(dev, rank, world, grp, last, groups, msda_stage, grad_bev, lat
     import torch.distributed as dist
 
     from vidar_b200 import ray_head, render, sca
-    bev, leaves, pred, grad_sigma, gemb, ce_grad, dv_grad = last
+    bev, leaves, pred, grad_sigma, gemb, ce_grad, dv_grad, _ = last
     full = sca_like_inputs(dev)
     ref_groups = [dict(plan=sca.unit_plan(1, 0, NUM_CAMS)[0], value=full["value"], loc=full["loc"], attn=full["attn"])]
     rbev, rleaves = msda_stage(ref_groups, None, 1)
@@ -907,7 +948,14 @@ def main():
     ap.add_argument("--workload", default="hotpath", choices=["hotpath", "pretrain"],
                     help="hotpath: BASELINE configs[1]+[2] (the headline line); pretrain: configs[3], the synthetic ViDAR-RN101 step "
                          "(--impl reference there = the same graph with the reference's eager torch formulas for MSDA / LatentRendering, on the GPU)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy (float32; "
+                         f"an output of more than {DUMP_SAMPLE} elements as a fixed, seeded sample of that many)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.workload, args.impl, args.gpus) != ("hotpath", "ours", 1):
+        ap.error("--dump-outputs writes the single-GPU hot path's outputs (--workload hotpath --impl ours --gpus 1)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.workload == "pretrain":
         run_pretrain(args)

@@ -66,16 +66,28 @@ def test_sca_fused_epilogue_equals_materialised_path(cuda):
 def test_sca_fused_rebatch_equals_reference_data_flow(cuda, bs):
     """SpatialCrossAttention's default path (device-side visible lists, offsets / logits once per pillar,
     rows reduced straight into the BEV slots: vidar_b200/sca.py) against the reference's rebatch /
-    index_add_ data flow on the same CUDA op -- output, input gradients and every parameter gradient."""
+    index_add_ data flow on the same CUDA op -- output, input gradients and every parameter gradient.
+
+    The two flows compute the sampling offsets with different GEMMs (once per pillar on the tensor cores, once per
+    (camera, pillar) row on cuBLAS).  Rounded differently, a sample within an ulp of a pixel-centre line lands on
+    either side of it, where d(out)/d(loc) jumps, and through `sampling_offsets` that one sample moves a whole row of
+    the query gradient.  So the query and that Linear's parameters are put on dyadic grids (query to 2^-6, weights to
+    2^-8), where both GEMMs are exact in fp32: both flows then sample at bit-identical locations."""
     m = build_attention(mc.SCA_CFG)
-    m.load_state_dict(mc.seeded_state(m, 10))
+    sd = mc.seeded_state(m, 10)
+    for k in ("deformable_attention.sampling_offsets.weight", "deformable_attention.sampling_offsets.bias"):
+        sd[k] = (sd[k] * 256).round() / 256
+    m.load_state_dict(sd)
     m.eval().to(cuda)
     assert m.fuse_rebatch
+    case = mc.sca_case(bs=bs)
+    for k in ("query", "query_pos"):
+        case[k] = (case[k] * 64).round() / 64
     res = []
     for fused in (True, False):
         m.fuse_rebatch = fused
         m.zero_grad(set_to_none=True)
-        out, gq, gkv = mc.run_module(m, "sca", mc.sca_case(bs=bs), device=cuda)
+        out, gq, gkv = mc.run_module(m, "sca", case, device=cuda)
         res.append([out, gq, gkv] + [p.grad.clone() for _, p in sorted(m.named_parameters())])
     names = ["out", "grad query", "grad key/value"] + [n for n, _ in sorted(m.named_parameters())]
     for a, b, w in zip(res[0], res[1], names):
