@@ -401,6 +401,39 @@ int vidar_nn_backward(const float* p1, const float* p2, const int64_t* lengths1,
                       const int64_t* lengths2, const int64_t* idx, const float* grad_dists,
                       float* grad_p1, float* grad_p2, int N, int P1, int P2, int D, void* stream);
 
+/* ------------------------------------------------------------------------------------
+ * (iv) point-cloud forecasting metrics, one segment = one (batch element, frame), N = bs * F
+ *   (ViDAR.forward_test, bevformer/detectors/vidar.py:389-502; get_rendered_pcds,
+ *   dense_heads/vidar_head_base.py:344-389; compute_chamfer_distance_inner,
+ *   utils/e2e_predictor_utils.py:146-184; clamp / _clamp / compute_ray_errors, utils/eval_utils.py:21-225)
+ *
+ * vidar_eval_gather: origin [bs, F, 3], points [bs, M, 3] (NaN padding), tindex [bs, M] (-1 padding),
+ *   gt_dist / pred_dist [bs, M] (metres; both NULL: the points themselves are the cloud of every
+ *   frame, pred = GT), pc_range_host: 6 host floats.  Rays of segment (b, t): tindex == t, gt_dist > 0,
+ *   and inside pc_range if within_grid.  Writes stably ordered (ray order) lists, padded to M:
+ *     pred_in, gt_in [N, M, 3]   predicted / GT points inside pc_range       counts[0*N + s], counts[1*N + s]
+ *     pred_sph [N, M, 3], pred_dhat [N, M]  (atan2(x,y), atan2(z,y), 1) of pred - origin with d_hat > 1e-2,
+ *                                            and d_hat                        counts[2*N + s]
+ *     gt_sph, gt_pts [N, M, 3]   the same for GT with d > 1e-2, and the GT point     counts[3*N + s]
+ *   counts [4, N] int64.  One block per segment.
+ *
+ * vidar_eval_ray_errors: nn_idx [N, Mg] = nearest pred_sph of every gt_sph (vidar_nn_forward);
+ *   cham_fwd [N, Mp] / cham_bwd [N, Mg] = squared NN distances pred_in -> gt_in and gt_in -> pred_in
+ *   (both NULL: Chamfer column 0).  pred_dhat is read with row stride Mp, gt_pts / nn_idx with Mg.
+ *   out [N, 4] fp64 = (chamfer-inner, l1, absrel, count of GT rays with d > 1e-2); count is -1 where
+ *   a clamped ray is degenerate (the reference raises RuntimeError) and -2 where a ray that meets the
+ *   eval box cannot be clamped into it (the reference's assert(touches_volume)).  Deterministic: one
+ *   block per segment, fixed-order fp64 sums, no atomics.
+ * ---------------------------------------------------------------------------------- */
+int vidar_eval_gather(const float* origin, const float* points, const float* tindex, const float* gt_dist,
+                      const float* pred_dist, const float* pc_range_host, int within_grid, float* pred_in,
+                      float* gt_in, float* pred_sph, float* pred_dhat, float* gt_sph, float* gt_pts,
+                      int64_t* counts, int bs, int M, int F, void* stream);
+
+int vidar_eval_ray_errors(const float* origin, const float* pred_dhat, const float* gt_pts,
+                          const int64_t* nn_idx, const float* cham_fwd, const float* cham_bwd,
+                          const int64_t* counts, double* out, int N, int Mp, int Mg, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

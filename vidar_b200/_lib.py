@@ -18,7 +18,7 @@ _lib = None
 _CTYPES = {
     "const float*": C.c_void_p, "float*": C.c_void_p, "const int64_t*": C.c_void_p,
     "const int32_t*": C.c_void_p, "int32_t*": C.c_void_p, "const unsigned char*": C.c_void_p, "unsigned char*": C.c_void_p, "int64_t*": C.c_void_p,
-    "unsigned long long*": C.c_void_p,
+    "unsigned long long*": C.c_void_p, "double*": C.c_void_p,
     "void*": C.c_void_p, "int": C.c_int, "float": C.c_float, "long long": C.c_longlong,
 }
 

@@ -16,7 +16,7 @@ CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libvidar_b200.so")
 STAMP = os.path.join(HERE, ".libvidar_b200.stamp")
 
-SOURCES = ["core.cu", "msda.cu", "linear_tc.cu", "dvr.cu", "latent_render.cu", "latent_proj.cu", "ray_head.cu", "sca_glue.cu", "knn.cu"]
+SOURCES = ["core.cu", "msda.cu", "linear_tc.cu", "dvr.cu", "latent_render.cu", "latent_proj.cu", "ray_head.cu", "sca_glue.cu", "knn.cu", "eval.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-O3", "-lineinfo", "-std=c++17",

@@ -31,7 +31,8 @@ nn_forward_kernel(const float* __restrict__ p1, const float* __restrict__ p2,
   const int L2 = len2 ? (int)len2[n] : P2;
   const int chunk = (L2 + splits - 1) / splits;
   const int j0 = blockIdx.y * chunk, j1 = min(L2, j0 + chunk);
-  if (j0 >= j1) return;
+  // nothing to do: no P2 points in this split, or (launched over an upper bound P1) no live p1 point
+  if (j0 >= j1 || (int)(blockIdx.x * kNnThreads) >= L1) return;
   float a[D];
   const bool live = i < L1;
 #pragma unroll

@@ -24,7 +24,7 @@ import numpy as np
 import torch
 import torch.nn.functional as F
 
-from . import bev_geometry, chamfer, ray_head
+from . import bev_geometry, chamfer, evaluation, ray_head
 
 
 def get_inside_mask(points, point_cloud_range):
@@ -212,6 +212,15 @@ class ViDARRayHead:
     # ------------------------------------------------------------------ decode (:662-752)
     def get_point_cloud_prediction(self, pred_dict, gt_points, start_idx, tgt_bev_h, tgt_bev_w, tgt_pc_range,
                                    img_metas=None, batched_origin_points=None):
+        batched_origin_points, batched_gt_points, gt_tindex, gt_dist, pred_dist = self._decode_rays(
+            pred_dict, gt_points, start_idx, tgt_bev_h, tgt_bev_w, tgt_pc_range, batched_origin_points)
+        pred_pcds = self.get_rendered_pcds(batched_origin_points, batched_gt_points, gt_tindex, gt_dist, pred_dist, tgt_pc_range)
+        gt_pcds = self.get_rendered_pcds(batched_origin_points, batched_gt_points, gt_tindex, gt_dist, gt_dist, tgt_pc_range)
+        return dict(pred_pcds=pred_pcds, gt_pcds=gt_pcds, origin=batched_origin_points)
+
+    # ------------------------------------------------------------------ evaluation (vidar.py:431-497)
+    def _decode_rays(self, pred_dict, gt_points, start_idx, tgt_bev_h, tgt_bev_w, tgt_pc_range, batched_origin_points):
+        """get_point_cloud_prediction's decode up to the padded per-ray distances (metres)."""
         bev_preds = pred_dict["next_bev_preds"].float()
         valid_frames = pred_dict["valid_frames"]
         pred_frame_num, inter_num, bs, token_num, num_height_pred = bev_preds.shape
@@ -225,7 +234,15 @@ class ViDARRayHead:
             pred_dist[b], gt_dist[b] = ray_head.decode_ray_depth(sigma[b], origin_grids[b], gt_grids[b], gt_tindex[b],
                                                                  self.ray_grid_step, self.ray_grid_num)
         scale = (tgt_pc_range[3] - tgt_pc_range[0]) / tgt_bev_w
-        pred_dist, gt_dist = pred_dist * scale, gt_dist * scale
-        pred_pcds = self.get_rendered_pcds(batched_origin_points, batched_gt_points, gt_tindex, gt_dist, pred_dist, tgt_pc_range)
-        gt_pcds = self.get_rendered_pcds(batched_origin_points, batched_gt_points, gt_tindex, gt_dist, gt_dist, tgt_pc_range)
-        return dict(pred_pcds=pred_pcds, gt_pcds=gt_pcds, origin=batched_origin_points)
+        return batched_origin_points, batched_gt_points, gt_tindex, gt_dist * scale, pred_dist * scale
+
+    def evaluate(self, pred_dict, gt_points, start_idx, tgt_bev_h, tgt_bev_w, tgt_pc_range, img_metas=None,
+                 batched_origin_points=None):
+        """get_point_cloud_prediction's decode, then every (sample, frame) metric on the device
+        (`evaluation.evaluate_rays`) -> forward_test's ret_dict {'frame.i': dict(count, chamfer_distance, l1_error,
+        absrel_error)}, summed over the batch like vidar.py:450-497.  One host sync, at the end."""
+        origin, points, tindex, gt_dist, pred_dist = self._decode_rays(
+            pred_dict, gt_points, start_idx, tgt_bev_h, tgt_bev_w, tgt_pc_range, batched_origin_points)
+        metrics = evaluation.evaluate_rays(origin, points, tindex, gt_dist, pred_dist, tgt_pc_range, origin.shape[1],
+                                           self.eval_within_grid)
+        return evaluation.ret_dict_from_metrics(metrics, start_idx)

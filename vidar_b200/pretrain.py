@@ -257,9 +257,10 @@ class SyntheticViDAR(nn.Module):
     """The pre-training graph of ViDAR-RN101 (3 history frames, 3 future frames, 5 predicted head frames)."""
 
     def __init__(self, num_cams=6, encoder_layers=6, decoder_layers=3, future_frames=3, history_frames=3,
-                 latent_layer=2, bev_hw=(BEV_H, BEV_W), ray_grid_num=512):
+                 latent_layer=2, bev_hw=(BEV_H, BEV_W), ray_grid_num=512, test_future_frames=6):
         super().__init__()
         self.num_cams, self.future_frames, self.history_frames = num_cams, future_frames, history_frames
+        self.test_future_frames = test_future_frames           # roll-outs of forward_test (cfg :18)
         self.bev_h, self.bev_w = bev_hw
         BEV_H, BEV_W = bev_hw          # noqa: N806  (shadows the module defaults below)
         self.backbone, self.neck = ImageBackbone(), FPN()
@@ -465,6 +466,44 @@ class SyntheticViDAR(nn.Module):
                 losses[f"frame.{i}.{k}"] = v
         self._mark("head+loss")
         return losses
+
+    # ---- one test forward (vidar.py:389-502) -> [ret_dict] of point-cloud forecasting metrics ----
+    def forward_test(self, img, lidar2img, gt_points, can_bus=None):
+        """img [bs, T, cams, 3, H, W], lidar2img [bs, cams, 4, 4] (host), gt_points: list over batch of [M, 4]
+        (x, y, z metric, frame index 0 = current .. test_future_frames).  Every frame is encoded (obtain_history_bev
+        in test mode, bevformer.py:217-232), the decoder rolls out `test_future_frames` times with a queue of length 1,
+        the head keeps prediction index `history_frames` (vidar_head_v1.py:234) and `ViDARRayHead.evaluate` scores
+        every (sample, frame).  Synthetic ego motion is the identity.  -> [ret_dict]."""
+        was_training = self.training
+        self.eval()
+        try:
+            with torch.no_grad():
+                bs, T = img.shape[:2]
+                can_bus = torch.zeros(bs, 18, device=img.device) if can_bus is None else can_bus
+                img_metas = [dict(lidar2img=np.asarray(lidar2img[b]), img_shape=[(img.shape[-2], img.shape[-1], 3)])
+                             for b in range(bs)]
+                prev_bev = None
+                for t in range(T):
+                    feats, shapes, lsi = self.extract_feat(img[:, t])
+                    self._mark(f"frame{t}.backbone")
+                    prev_bev = self.encode(feats, shapes, lsi, img_metas, can_bus, prev_bev)
+                    self._mark(f"frame{t}.encoder")
+                next_bev_feats = [prev_bev.unsqueeze(0).repeat(len(self.bev_pred_head), 1, 1, 1)]
+                prev_bev_input = prev_bev.unsqueeze(1)
+                for _ in range(self.test_future_frames):
+                    pred_feat, last = self.decode_future(prev_bev_input, can_bus)
+                    next_bev_feats.append(pred_feat)
+                    prev_bev_input = last.unsqueeze(1)
+                self._mark("future_decoder")
+                next_bev_preds = self.forward_head(torch.stack(next_bev_feats, 0))
+                pred_dict = dict(next_bev_preds=next_bev_preds[:, :, self.history_frames],
+                                 valid_frames=list(range(1 + self.test_future_frames)))
+                self._mark("head")
+                ret_dict = self.ray_head.evaluate(pred_dict, gt_points, 0, self.bev_h, self.bev_w, PC_RANGE)
+                self._mark("metrics")
+        finally:
+            self.train(was_training)
+        return [ret_dict]
 
 
 # ------------------------------------------------------------------------------------------------
