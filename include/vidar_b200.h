@@ -434,6 +434,31 @@ int vidar_eval_ray_errors(const float* origin, const float* pred_dhat, const flo
                           const int64_t* nn_idx, const float* cham_fwd, const float* cham_bwd,
                           const int64_t* counts, double* out, int N, int Mp, int Mg, void* stream);
 
+/* ------------------------------------------------------------------------------------
+ * (v) ego motion (csrc/ego.cu)
+ *
+ * vidar_bev_rotate_forward: the previous BEV rotated like PerceptionTransformer.get_bev_features
+ *   (bevformer/modules/transformer.py:136-149): torchvision.transforms.functional.rotate(img[C,H,W],
+ *   angle, center) with nearest sampling, expand=False and zero fill, per sample.
+ *   src, dst [bs, H*W, C] channel-last (must not alias); theta_host [bs, 3, 2] host floats = the
+ *   rescaled affine matrix θᵀ / [W/2, H/2] of torchvision's _gen_affine_grid (rows x, y, 1).
+ *   One warp per output cell; forward only.
+ *
+ * vidar_ego_align_points: ViDARHeadV1._get_reference_gt_points (dense_heads/vidar_head_v1.py:94-148)
+ *   without its masks.  points [N, 4] (x, y, z, frame) packed over the batch, offsets_host [bs + 1]
+ *   (N = offsets_host[bs]); slot_of_frame_host [num_frames] = the slot s of frame f, or -1;
+ *   src_to_tgt_host [bs, S, 4, 4] host floats (row-vector convention p' = p @ M).
+ *   out_points [N, 4] = ([x y z 1] @ M[b, s], s) for points of a frame with a slot, else
+ *   (NaN, NaN, NaN, -1), in input order; origins [bs, S, 3] = [0 0 0 1] @ M[b, s].
+ *   One thread per point; points and out_points may be NULL when N == 0.
+ * ---------------------------------------------------------------------------------- */
+int vidar_bev_rotate_forward(const float* src, const float* theta_host, float* dst, int bs, int H, int W, int C,
+                             void* stream);
+
+int vidar_ego_align_points(const float* points, const int64_t* offsets_host, const int32_t* slot_of_frame_host,
+                           int num_frames, const float* src_to_tgt_host, float* out_points, float* origins, int bs,
+                           int S, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -3,8 +3,8 @@
   get_reference_points  BEVFormerEncoder.get_reference_points  (modules/encoder.py:53-92)
   point_sampling        BEVFormerEncoder.point_sampling        (modules/encoder.py:94-156) -- CUDA
                         kernel csrc/sca_glue.cu instead of a 61 MB repeat + batched matmul + masks
-  coords_to_voxel_grids / get_bev_grids / get_bev_grids_3d
-                        bevformer/utils/e2e_predictor_utils.py:36-45, 48-83
+  coords_to_voxel_grids / get_bev_grids / get_bev_grids_3d / bev_grids_to_coordinates / bev_coords_to_grids
+                        bevformer/utils/e2e_predictor_utils.py:8-45, 48-83
 Index/grid generation is plain torch on the target device (no arithmetic worth a kernel).
 """
 import copy
@@ -68,6 +68,26 @@ def get_bev_grids(H, W, bs=1, device="cuda", dtype=torch.float, offset=0.5):
     ref_y, ref_x = torch.meshgrid(ys, xs, indexing="ij")
     ref = torch.stack((ref_x.reshape(-1)[None] / W, ref_y.reshape(-1)[None] / H), -1)
     return ref.repeat(bs, 1, 1)
+
+
+def bev_grids_to_coordinates(ref_grids, pc_range):
+    """e2e_predictor_utils.py:8-14: [0, 1] grids -> metric x, y."""
+    c = copy.deepcopy(ref_grids)
+    c[..., 0:1] = c[..., 0:1] * (pc_range[3] - pc_range[0]) + pc_range[0]
+    c[..., 1:2] = c[..., 1:2] * (pc_range[4] - pc_range[1]) + pc_range[1]
+    return c
+
+
+def bev_coords_to_grids(ref_coords, bev_h, bev_w, pc_range):
+    """e2e_predictor_utils.py:16-33: metric x, y -> ([-1, 1] grids, mask of the cells off the border)."""
+    g = copy.deepcopy(ref_coords)
+    g[..., 0] = (g[..., 0] - pc_range[0]) / (pc_range[3] - pc_range[0])
+    g[..., 1] = (g[..., 1] - pc_range[1]) / (pc_range[4] - pc_range[1])
+    g = g * 2 - 1.
+    x_min, x_max = 0.5 / bev_w * 2 - 1, (bev_w - 0.5) / bev_w * 2 - 1
+    y_min, y_max = 0.5 / bev_h * 2 - 1, (bev_h - 0.5) / bev_h * 2 - 1
+    valid = (g[..., 0:1] > x_min) & (g[..., 0:1] < x_max) & (g[..., 1:2] > y_min) & (g[..., 1:2] < y_max)
+    return g, valid
 
 
 def get_bev_grids_3d(H, W, Z, bs=1, device="cuda", dtype=torch.float):

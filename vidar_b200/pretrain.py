@@ -35,7 +35,7 @@ import torch
 import torch.nn as nn
 import torch.nn.functional as F
 
-from . import bev_geometry, sca, sharding, synthetic
+from . import bev_geometry, ego, sca, sharding, synthetic
 from . import modules as _modules  # noqa: F401  (registers the attention classes)
 from .head import ViDARRayHead
 from .modules.deform_attn import _linear
@@ -235,19 +235,22 @@ class DecoderLayer(nn.Module):
         return sharding.all_gather_rows(q[0], Q, group, grad="sum")[None]
 
 
-def run_decoder(layers, query, prev, bev_pos, ref, bev_shapes, bev_lsi, group=None):
+def run_decoder(layers, query, prev, bev_pos, ref, bev_shapes, bev_lsi, group=None, ref_points=None):
     """The future-BEV decoder stack -> (outputs of every layer stacked [inter, bs, Q, C] for the head, last output for
-    the next future frame).  `group`: row-sharded layers (`DecoderLayer.forward_rows`); the stacked outputs are then
+    the next future frame).  `ref`: the self-attention's reference points in the target frame (`tgt_points`),
+    `ref_points`: the cross-attention's in the previous frame (vidar_decoder.py:205-262); None = `ref`, the identity
+    ego motion.  `group`: row-sharded layers (`DecoderLayer.forward_rows`); the stacked outputs are then
     (like the returned last output) views for replicated consumers (`sharding.replicated_view`)."""
     inter = []
+    ref_points = ref if ref_points is None else ref_points
     if group is None:
         for layer in layers:
-            query = layer(query, prev, bev_pos, ref, ref, bev_shapes, bev_lsi)
+            query = layer(query, prev, bev_pos, ref, ref_points, bev_shapes, bev_lsi)
             inter.append(query)
         return torch.stack(inter), inter[-1]
     query, prev, bev_pos = (sharding.sum_grad(t, group) for t in (query, prev, bev_pos))
     for layer in layers:
-        query = layer.forward_rows(query, prev, bev_pos, ref, ref, bev_shapes, bev_lsi, group)
+        query = layer.forward_rows(query, prev, bev_pos, ref, ref_points, bev_shapes, bev_lsi, group)
         inter.append(sharding.replicated_view(query, group))
     # the caller's use of the last output (next frame's `prev`, which passes through sum_grad again) is replicated too
     return torch.stack(inter), inter[-1]
@@ -257,10 +260,15 @@ class SyntheticViDAR(nn.Module):
     """The pre-training graph of ViDAR-RN101 (3 history frames, 3 future frames, 5 predicted head frames)."""
 
     def __init__(self, num_cams=6, encoder_layers=6, decoder_layers=3, future_frames=3, history_frames=3,
-                 latent_layer=2, bev_hw=(BEV_H, BEV_W), ray_grid_num=512, test_future_frames=6):
+                 latent_layer=2, bev_hw=(BEV_H, BEV_W), ray_grid_num=512, test_future_frames=6,
+                 history_queue_length=None, rotate_center=(100, 100)):
         super().__init__()
         self.num_cams, self.future_frames, self.history_frames = num_cams, future_frames, history_frames
         self.test_future_frames = test_future_frames           # roll-outs of forward_test (cfg :18)
+        # ego motion (`img_metas` path): GT queue index of the current frame (ViDARHeadV1.history_queue_length) and
+        # the previous-BEV rotation centre in cells (PerceptionTransformer.rotate_center)
+        self.history_queue_length = history_frames if history_queue_length is None else history_queue_length
+        self.rotate_center = list(rotate_center)
         self.bev_h, self.bev_w = bev_hw
         BEV_H, BEV_W = bev_hw          # noqa: N806  (shadows the module defaults below)
         self.backbone, self.neck = ImageBackbone(), FPN()
@@ -365,7 +373,10 @@ class SyntheticViDAR(nn.Module):
         return feats, spatial_shapes, lsi
 
     # ---- BEV encoder (transformer.py:102-193 + encoder.py:159-253) ----
-    def encode(self, feats, spatial_shapes, lsi, img_metas, can_bus, prev_bev):
+    def encode(self, feats, spatial_shapes, lsi, img_metas, can_bus, prev_bev, ego_motion=False):
+        """`ego_motion`: `img_metas` are the reference's per-frame metas; the previous BEV is rotated by
+        `can_bus[-1]` degrees and the previous half of TSA's reference points is shifted by the ego translation
+        (transformer.py:120-157, encoder.py:203-216).  Otherwise `can_bus` is used as given (zeros: no ego motion)."""
         bs = feats.shape[2]
         dev = feats.device
         BEV_H, BEV_W = self.bev_h, self.bev_w          # noqa: N806
@@ -375,7 +386,14 @@ class SyntheticViDAR(nn.Module):
         ref_2d = bev_geometry.get_reference_points(BEV_H, BEV_W, dim="2d", bs=bs, device=dev)
         ref_cam, bev_mask = bev_geometry.point_sampling(ref_3d, PC_RANGE, img_metas)
         Q = BEV_H * BEV_W
-        hybrid = torch.stack([ref_2d, ref_2d], 1).reshape(bs * 2, Q, 1, 2)          # can_bus zeros: no ego shift
+        if ego_motion and prev_bev is not None:
+            grid_length = ((PC_RANGE[4] - PC_RANGE[1]) / BEV_H, (PC_RANGE[3] - PC_RANGE[0]) / BEV_W)
+            shift = ref_2d.new_tensor(ego.bev_shift(img_metas, grid_length, BEV_H, BEV_W))
+            prev_bev = ego.rotate_prev_bev(prev_bev, [m["can_bus"][-1] for m in img_metas], self.rotate_center,
+                                           BEV_H, BEV_W)
+            hybrid = torch.stack([ref_2d + shift[:, None, None, :], ref_2d], 1).reshape(bs * 2, Q, 1, 2)
+        else:
+            hybrid = torch.stack([ref_2d, ref_2d], 1).reshape(bs * 2, Q, 1, 2)      # can_bus zeros: no ego shift
         bev_shapes = torch.tensor([[BEV_H, BEV_W]], device=dev)
         bev_lsi = torch.tensor([0], device=dev)
         rows_mode = getattr(self, "row_sharded", False)
@@ -397,21 +415,26 @@ class SyntheticViDAR(nn.Module):
         return query
 
     # ---- future decoder (vidar_head_base.py:125-173) ----
-    def decode_future(self, prev_bev_input, future_can_bus):
+    def decode_future(self, prev_bev_input, future_can_bus, tgt_points=None, ref_points=None):
+        """`future_can_bus` [bs, 18]: all 18 dims of `future_can_bus[k]` go through the future MLP (the reference
+        selects `can_bus_dims=(0, 1, 2, 17)`; this harness keeps its 18-input MLP).  `tgt_points` / `ref_points`
+        [bs, Q, 1, 2]: the decoder's self- / cross-attention reference points (`ego.align_bev_coordinates`);
+        None = the untransformed BEV grid (identity ego motion)."""
         bs = prev_bev_input.shape[0]
         dev = prev_bev_input.device
         BEV_H, BEV_W = self.bev_h, self.bev_w          # noqa: N806
         bev_pos = self.future_positional_encoding(bs)
         query = self.future_bev_embedding.weight[None] + self.future_can_bus_mlp(future_can_bus)[:, None]
         prev = (prev_bev_input + self.prev_frame_embedding[None, :, None, :]).view(bs, -1, EMBED)
-        ref = bev_geometry.get_reference_points(BEV_H, BEV_W, dim="2d", bs=bs, device=dev)      # identity ego motion
+        ref = bev_geometry.get_reference_points(BEV_H, BEV_W, dim="2d", bs=bs, device=dev) if tgt_points is None else tgt_points
         bev_shapes = torch.tensor([[BEV_H, BEV_W]], device=dev)
         bev_lsi = torch.tensor([0], device=dev)
         rows_mode = getattr(self, "row_sharded", False)
         if rows_mode and (bs != 1 or query.shape[1] % torch.distributed.get_world_size(self.process_group) != 0):
             raise RuntimeError("row-sharded decoder: needs bs == 1 and BEV rows divisible by the group size")
         # -> ([inter, bs, Q, C] for the head, the last layer's output for the next future frame)
-        return run_decoder(self.decoder, query, prev, bev_pos, ref, bev_shapes, bev_lsi, self.process_group if rows_mode else None)
+        return run_decoder(self.decoder, query, prev, bev_pos, ref, bev_shapes, bev_lsi, self.process_group if rows_mode else None,
+                           ref_points=ref_points)
 
     def forward_head(self, next_bev_feats):
         """vidar_head_v1.py:64-92: [frames, inter, bs, Q, C] -> [frames, inter, pred_frame, bs, Q, heights]."""
@@ -425,11 +448,114 @@ class SyntheticViDAR(nn.Module):
             preds.append(p.permute(0, 4, 1, 2, 3).contiguous())
         return torch.stack(preds, 1)
 
+    # ---- ego motion (img_metas path) ----
+    @staticmethod
+    def _frame_metas(img_metas, t, lidar2img, img):
+        """The reference's metas of input frame t for every sample; `lidar2img` / `img_shape` default to the
+        call's arguments where a meta lacks them."""
+        out = []
+        for b, m in enumerate(img_metas):
+            m = dict(m[t])
+            if "lidar2img" not in m:
+                m["lidar2img"] = np.asarray(lidar2img[b])
+            m.setdefault("img_shape", [(img.shape[-2], img.shape[-1], 3)])
+            out.append(m)
+        return out
+
+    def _encode_ego(self, img, img_metas, lidar2img, t, prev_bev):
+        """One frame of obtain_history_bev (bevformer.py:158-189): `prev_bev_exists` of sample 0 resets the
+        recurrence, `can_bus` of the frame feeds the query MLP, rotation and shift."""
+        metas = self._frame_metas(img_metas, t, lidar2img, img)
+        if not metas[0]["prev_bev_exists"]:
+            prev_bev = None
+        feats, shapes, lsi = self.extract_feat(img[:, t])
+        can_bus = img.new_tensor(np.array([m["can_bus"] for m in metas], np.float64)).float()
+        return self.encode(feats, shapes, lsi, metas, can_bus, prev_bev, ego_motion=True), metas
+
+    def _roll_out_ego(self, ref_bev, cur_metas, num_future):
+        """The future roll-out of vidar.py:316-363 with a queue of one previous BEV: the decoder's query grid in
+        each future frame and its position in the previous frame (`ego.align_bev_coordinates`), the future
+        `can_bus`, and the `ref_to_history` queue update -> list of [inter, bs, Q, C]."""
+        next_bev_feats = [ref_bev.unsqueeze(0).repeat(len(self.bev_pred_head), 1, 1, 1)]
+        prev_bev_input = ref_bev.unsqueeze(1)
+        ref_to_history = ego.history_ref_to_previous_transform(prev_bev_input, prev_bev_input.shape[1],
+                                                               [[m] for m in cur_metas])
+        for k in range(1, num_future + 1):
+            tgt, aligned, ref2future = ego.align_bev_coordinates(k, ref_to_history, cur_metas, self.bev_h, self.bev_w,
+                                                                 PC_RANGE)
+            future_can_bus = ref_bev.new_tensor(np.array([m["future_can_bus"][k] for m in cur_metas], np.float64))
+            pred_feat, last = self.decode_future(prev_bev_input, future_can_bus, tgt_points=tgt.unsqueeze(2),
+                                                 ref_points=aligned)
+            next_bev_feats.append(pred_feat)
+            prev_bev_input = torch.cat([prev_bev_input, last.unsqueeze(1)], 1)[:, 1:]
+            ref_to_history = torch.cat([ref_to_history, ref2future.unsqueeze(1)], 1)[:, 1:].contiguous()
+        return next_bev_feats
+
+    def _forward_train_ego(self, img, lidar2img, gt_points, img_metas):
+        bs, T = img.shape[:2]
+        prev_bev = None
+        with torch.no_grad():                                                        # obtain_history_bev
+            for t in range(T - 1):
+                prev_bev, _ = self._encode_ego(img, img_metas, lidar2img, t, prev_bev)
+                self._mark(f"hist{t}.encoder")
+        ref_bev, cur_metas = self._encode_ego(img, img_metas, lidar2img, T - 1, prev_bev)
+        self._mark("cur.encoder")
+        next_bev_feats = self._roll_out_ego(ref_bev, cur_metas, self.future_frames)
+        self._mark("future_decoder")
+        next_bev_preds = self.forward_head(torch.stack(next_bev_feats, 0))            # [F, inter, pred_frame, bs, Q, 16]
+        # ViDARHeadV1.loss (vidar_head_v1.py:150-219)
+        valid_frames = np.arange(1 + self.future_frames)
+        hq, ph = self.history_queue_length, self.history_frames
+        start_frames, tgt_frames = valid_frames + hq - ph, valid_frames + hq
+        frame_idx_for_loss = (np.arange(self.pred_frame_num) if ego.full_prev_bev_exists(img_metas)
+                              else [ph] * self.pred_frame_num)
+        n_w = len(self.ray_head.loss_weight)
+        losses = {}
+        for idx, i in enumerate(frame_idx_for_loss):
+            pts, origins = ego.align_gt_points(gt_points, start_frames + i, tgt_frames, cur_metas)
+            lw = np.array([[1]] + [[0]] * (n_w - 1)) if i != ph else self.ray_head.loss_weight
+            pred_dict = dict(next_bev_preds=next_bev_preds[:, :, i], valid_frames=list(range(len(valid_frames))))
+            ld = self.ray_head.loss(pred_dict, pts, 0, self.bev_h, self.bev_w, PC_RANGE, pred_frame_num=len(valid_frames),
+                                    batched_origin_points=origins, loss_weight=lw)
+            w = self.per_frame_loss_weight[i] * (idx == i)
+            for k, v in ld.items():
+                losses[f"frame.{idx}.{k}"] = v * w
+        self._mark("head+loss")
+        return losses
+
+    def _forward_test_ego(self, img, lidar2img, gt_points, img_metas):
+        bs, T = img.shape[:2]
+        prev_bev = None
+        for t in range(T):
+            prev_bev, cur_metas = self._encode_ego(img, img_metas, lidar2img, t, prev_bev)
+            self._mark(f"frame{t}.encoder")
+        next_bev_feats = self._roll_out_ego(prev_bev, cur_metas, self.test_future_frames)
+        self._mark("future_decoder")
+        next_bev_preds = self.forward_head(torch.stack(next_bev_feats, 0))
+        valid_frames = np.arange(1 + self.test_future_frames)
+        frames = valid_frames + self.history_queue_length                   # vidar_head_v1.py:237-241: src = tgt
+        pts, origins = ego.align_gt_points(gt_points, frames, frames, cur_metas)
+        pred_dict = dict(next_bev_preds=next_bev_preds[:, :, self.history_frames], valid_frames=list(valid_frames))
+        self._mark("head")
+        ret_dict = self.ray_head.evaluate(pred_dict, pts, 0, self.bev_h, self.bev_w, PC_RANGE, batched_origin_points=origins)
+        self._mark("metrics")
+        return ret_dict
+
     # ---- one training forward (vidar.py:239-387) -> dict of losses ----
-    def forward_train(self, img, lidar2img, gt_points, can_bus=None):
+    def forward_train(self, img, lidar2img, gt_points, can_bus=None, img_metas=None):
         """img [bs, T, cams, 3, H, W] (T-1 history frames + current), lidar2img: host array [bs, cams, 4, 4]
-        (it lives in `img_metas` in the reference), gt_points: list over batch of [M, 4] (x, y, z metric,
-        frame index 0 = current .. future_frames)."""
+        (it lives in `img_metas` in the reference), gt_points: list over batch of [M, 4] (x, y, z metric, frame).
+
+        img_metas None: no ego motion; GT frame index 0 = current .. future_frames.
+        img_metas given (the reference's metas, list over the batch of lists over the T input frames, e.g.
+        `synthetic.ego_queue`): per-frame `can_bus`, `prev_bev_exists`, previous-BEV rotation and shift, the future
+        decoder aligned to the future poses and the ViDARHeadV1 loss loop with GT moved into each target frame.
+        GT frame index is then the reference's queue index: 0 = the oldest history frame, `history_queue_length`
+        (default T - 1) = the current frame.  Passing both `can_bus` and `img_metas` raises ValueError."""
+        if img_metas is not None:
+            if can_bus is not None:
+                raise ValueError("forward_train: pass either can_bus or img_metas (whose frames carry can_bus), not both")
+            return self._forward_train_ego(img, lidar2img, gt_points, img_metas)
         bs, T = img.shape[:2]
         dev = img.device
         can_bus = torch.zeros(bs, 18, device=dev) if can_bus is None else can_bus
@@ -468,16 +594,24 @@ class SyntheticViDAR(nn.Module):
         return losses
 
     # ---- one test forward (vidar.py:389-502) -> [ret_dict] of point-cloud forecasting metrics ----
-    def forward_test(self, img, lidar2img, gt_points, can_bus=None):
+    def forward_test(self, img, lidar2img, gt_points, can_bus=None, img_metas=None):
         """img [bs, T, cams, 3, H, W], lidar2img [bs, cams, 4, 4] (host), gt_points: list over batch of [M, 4]
-        (x, y, z metric, frame index 0 = current .. test_future_frames).  Every frame is encoded (obtain_history_bev
-        in test mode, bevformer.py:217-232), the decoder rolls out `test_future_frames` times with a queue of length 1,
-        the head keeps prediction index `history_frames` (vidar_head_v1.py:234) and `ViDARRayHead.evaluate` scores
-        every (sample, frame).  Synthetic ego motion is the identity.  -> [ret_dict]."""
+        (x, y, z metric, frame).  Every frame is encoded (obtain_history_bev in test mode, bevformer.py:217-232), the
+        decoder rolls out `test_future_frames` times with a queue of length 1, the head keeps prediction index
+        `history_frames` (vidar_head_v1.py:234) and `ViDARRayHead.evaluate` scores every (sample, frame).
+
+        img_metas None: identity ego motion; GT frame index 0 = current .. test_future_frames.
+        img_metas given (as in `forward_train`): the ego-motion roll-out, and the GT of every evaluated frame in its
+        own coordinates with its sensor origin; GT frame index is the reference's queue index (0 = the oldest
+        history frame, `history_queue_length` = the current frame).  -> [ret_dict]."""
+        if img_metas is not None and can_bus is not None:
+            raise ValueError("forward_test: pass either can_bus or img_metas (whose frames carry can_bus), not both")
         was_training = self.training
         self.eval()
         try:
             with torch.no_grad():
+                if img_metas is not None:
+                    return [self._forward_test_ego(img, lidar2img, gt_points, img_metas)]
                 bs, T = img.shape[:2]
                 can_bus = torch.zeros(bs, 18, device=img.device) if can_bus is None else can_bus
                 img_metas = [dict(lidar2img=np.asarray(lidar2img[b]), img_shape=[(img.shape[-2], img.shape[-1], 3)])
@@ -525,6 +659,20 @@ def synthetic_sample(device, frames=4, cams=6, img_hw=synthetic.IMG_HW, rays_per
                     p[:, 2] / HEIGHTS * (PC_RANGE[5] - PC_RANGE[2]) + PC_RANGE[2]], -1)
     pts.append(torch.from_numpy(np.concatenate([xyz, tindex[0][:, None]], -1).astype(np.float32)).to(device))
     return dict(img=img, lidar2img=lidar2img, gt_points=pts)
+
+
+def synthetic_ego_sample(device, frames=4, cams=6, img_hw=synthetic.IMG_HW, rays_per_frame=10000, future_frames=4, seed=0,
+                         bs=1, speed=8.0, yaw_rate=0.15):
+    """A moving-ego sample: N(0,1) images, `synthetic.ego_queue` metas (the reference's `img_metas`) and the LiDAR
+    returns of its static world, indexed like the reference's queue (0 = oldest history frame, frames - 1 = current,
+    then `future_frames` future frames)."""
+    g = torch.Generator(device=device).manual_seed(seed)
+    img = torch.randn(bs, frames, cams, 3, img_hw[0], img_hw[1], device=device, generator=g)
+    q = synthetic.ego_queue(bs=bs, T=frames, future=future_frames, speed=speed, yaw_rate=yaw_rate, seed=seed,
+                            points_per_frame=rays_per_frame, cams=cams, img_hw=img_hw)
+    lidar2img = np.stack([m[frames - 1]["lidar2img"] for m in q["img_metas"]]).astype(np.float32)
+    return dict(img=img, lidar2img=lidar2img, img_metas=q["img_metas"],
+                gt_points=[torch.from_numpy(p).to(device) for p in q["gt_points"]])
 
 
 def train_step(model, optimizer, sample, group=None, record=False):

@@ -5,6 +5,8 @@ and no checkpoint in this tier, so the workload generators are part of the packa
   sca_like_inputs    configs[1]: MSDA operands at the SpatialCrossAttention shape
   dvr_inputs_lidar   configs[2]: sigma volume + LiDAR-like rays
   camera_rig         cfg4: a nuScenes-like 6-camera rig (lidar2img matrices) for point_sampling
+  ego_queue          a vehicle on a curved path through a static world: the reference's `img_metas` of one
+                     training / test queue and the LiDAR returns of every frame
 """
 import math
 
@@ -105,3 +107,134 @@ def camera_rig(cams=6, img_hw=(900, 1600), f=1266.0, pp=(816.0, 491.0), cam_heig
         E[:3, 3] = -R @ pos
         mats.append(K @ E)
     return torch.from_numpy(np.stack(mats, 0).astype(np.float32))
+
+
+def _yaw_matrix(yaw):
+    c, s = math.cos(yaw), math.sin(yaw)
+    return np.array([[c, -s, 0.0], [s, c, 0.0], [0.0, 0.0, 1.0]])
+
+
+def _yaw_quaternion(yaw):
+    return np.array([math.cos(yaw / 2), 0.0, 0.0, math.sin(yaw / 2)])          # (w, x, y, z)
+
+
+def _transform_matrix(translation, rotation, inverse=False):
+    """nuscenes.utils.geometry_utils.transform_matrix with a rotation matrix in place of the quaternion."""
+    m = np.eye(4)
+    if inverse:
+        m[:3, :3] = rotation.T
+        m[:3, 3] = -rotation.T @ np.asarray(translation)
+    else:
+        m[:3, :3] = rotation
+        m[:3, 3] = translation
+    return m
+
+
+def ego_queue(bs=1, T=4, future=4, speed=8.0, yaw_rate=0.15, seed=0, dt=0.5, points_per_frame=2000, cams=6,
+              img_hw=IMG_HW, world_points=None, max_range=60.0):
+    """A vehicle drives a curved path (`speed` m/s, `yaw_rate` rad/s, one frame every `dt` s) through a static
+    synthetic world.  Queue frame i = 0 .. T - 1 + future: T - 1 history frames, the current frame T - 1 and
+    `future` future frames, like `previous_queue[:-1] + future_queue` of
+    projects/mmdet3d_plugin/datasets/nuscenes_vidar_dataset_v1.py.  Every sample starts from its own pose and
+    speed.
+
+    -> dict(img_metas, gt_points): img_metas[b][t] for the T input frames with the keys and meanings of
+    `union2one` (nuscenes_vidar_dataset_v1.py:40-200) and `get_data_info` (nuscenes_dataset.py:153-225):
+    `can_bus` (18: deltas of position and yaw against the previous frame, the first frame zeroed),
+    `lidar2global_rotation`, `prev_bev_exists`, `ref_lidar_to_cur_lidar`, `lidar2img`, `img_shape`, the poses;
+    the current frame additionally `future_can_bus`, `future2ref_lidar_transform`, `ref2future_lidar_transform`,
+    `total_cur2ref_lidar_transform` and `total_ref2cur_lidar_transform` (row-vector convention, p' = p @ M).
+    gt_points[b]: float32 [M, 4] = the LiDAR returns of the static world from each frame's pose, in that frame's
+    LiDAR coordinates, last column = queue index.  Here the poses are synthetic in place of nuScenes records."""
+    rng = np.random.default_rng(seed)
+    world_points = max(40000, 4 * points_per_frame) if world_points is None else world_points
+    n_frames = T + future
+    lidar2img = camera_rig(cams, seed=seed).numpy().astype(np.float64)
+    l2e_t, l2e_yaw = np.array([0.94, 0.0, 1.84]), math.pi / 2          # LiDAR mounted like nuScenes': yawed 90 deg
+    l2e_r = _yaw_matrix(l2e_yaw)
+    metas_all, pts_all = [], []
+    for b in range(bs):
+        yaw0 = rng.uniform(-math.pi, math.pi)
+        v = speed * rng.uniform(0.8, 1.2)
+        w = yaw_rate * rng.uniform(0.8, 1.2) * (1 if b % 2 == 0 else -1)
+        pos = np.array([rng.uniform(300, 1800), rng.uniform(300, 1800), 0.0])
+        poses = []                                                          # ego2global (translation, yaw)
+        for _ in range(n_frames):
+            poses.append((pos.copy(), yaw0))
+            pos = pos + v * dt * np.array([math.cos(yaw0 + w * dt / 2), math.sin(yaw0 + w * dt / 2), 0.0])
+            yaw0 = yaw0 + w * dt
+        centre = np.mean([p for p, _ in poses], 0)
+        world = np.concatenate([centre[None, :2] + rng.uniform(-max_range - 40, max_range + 40, (world_points, 2)),
+                                rng.uniform(-1.6, 2.5, (world_points, 1))], 1)
+        raw = []                                                            # get_data_info: per-frame metas
+        for t, yaw in poses:
+            patch_angle = math.degrees(yaw) % 360.0
+            can_bus = np.zeros(18)
+            can_bus[:3] = t
+            can_bus[3:7] = _yaw_quaternion(yaw)
+            can_bus[12] = w
+            can_bus[13] = v
+            can_bus[-2] = patch_angle / 180 * np.pi
+            can_bus[-1] = patch_angle
+            raw.append(dict(ego2global_translation=t, ego2global_rotation=_yaw_quaternion(yaw),
+                            lidar2ego_translation=l2e_t, lidar2ego_rotation=_yaw_quaternion(l2e_yaw),
+                            lidar2global_rotation=_yaw_matrix(yaw) @ l2e_r, scene_token=f"synthetic-{seed}-{b}",
+                            can_bus=can_bus, lidar2img=lidar2img, img_shape=[(img_hw[0], img_hw[1], 3)] * cams,
+                            _e2g=(t, _yaw_matrix(yaw))))
+        # union2one 1: every frame <-> the reference (current) frame, and the points of every frame
+        ref_t, ref_r = raw[T - 1]["_e2g"]
+        ref_e2g, ref_g2e = _transform_matrix(ref_t, ref_r), _transform_matrix(ref_t, ref_r, inverse=True)
+        ref_l2e, ref_e2l = _transform_matrix(l2e_t, l2e_r), _transform_matrix(l2e_t, l2e_r, inverse=True)
+        cur2ref, ref2cur, pts = [], [], []
+        for i, m in enumerate(raw):
+            t, r = m["_e2g"]
+            e2g, g2e = _transform_matrix(t, r), _transform_matrix(t, r, inverse=True)
+            l2e, e2l = _transform_matrix(l2e_t, l2e_r), _transform_matrix(l2e_t, l2e_r, inverse=True)
+            cur2ref.append(l2e.T @ e2g.T @ ref_g2e.T @ ref_e2l.T)
+            ref2cur.append(ref_l2e.T @ ref_e2g.T @ g2e.T @ e2l.T)
+            # LiDAR returns: the world in this frame's LiDAR coordinates, within range
+            g2l = e2l @ g2e
+            local = world @ g2l[:3, :3].T + g2l[:3, 3]
+            keep = np.flatnonzero((np.abs(local[:, 0]) < max_range) & (np.abs(local[:, 1]) < max_range)
+                                  & (np.hypot(local[:, 0], local[:, 1]) > 2.0))
+            keep = rng.choice(keep, min(points_per_frame, keep.size), replace=False)
+            pts.append(np.concatenate([local[keep], np.full((keep.size, 1), i)], 1))
+        # union2one 2: can_bus deltas of the previous frames, future can_bus and transforms
+        metas, prev_pos, prev_angle = [], None, None
+        for i in range(T):
+            m = {k: v_ for k, v_ in raw[i].items() if k != "_e2g"}
+            m["can_bus"] = raw[i]["can_bus"].copy()
+            if i == 0:
+                m["prev_bev_exists"] = False
+                prev_pos, prev_angle = m["can_bus"][:3].copy(), m["can_bus"][-1]
+                m["can_bus"][:3], m["can_bus"][-1] = 0, 0
+            else:
+                m["prev_bev_exists"] = True
+                tmp_pos, tmp_angle = m["can_bus"][:3].copy(), m["can_bus"][-1]
+                m["can_bus"][:3], m["can_bus"][-1] = tmp_pos - prev_pos, tmp_angle - prev_angle
+                prev_pos, prev_angle = tmp_pos, tmp_angle
+            m["ref_lidar_to_cur_lidar"] = ref2cur[i]
+            metas.append(m)
+        future_can_bus, future2ref, ref2future, ref_can_bus = [], [], [], None
+        for i in range(future + 1):
+            future2ref.append(cur2ref[i + T - 1])
+            ref2future.append(ref2cur[i + T - 1])
+            c = raw[i + T - 1]["can_bus"].copy()
+            if i == 0:
+                ref_can_bus = c.copy()
+                c[:3], c[-1] = 0, 0
+            else:
+                p = np.array([0, 0, 0, 1]).reshape(1, 4) @ future2ref[-1] @ ref2future[-2]
+                angle = c[-1] - ref_can_bus[-1]
+                ref_can_bus = c.copy()
+                c[:3], c[-1] = p[:, :3], angle
+            future_can_bus.append(c)
+        cur = metas[T - 1]
+        cur["future_can_bus"] = np.array(future_can_bus)
+        cur["future2ref_lidar_transform"] = np.array(future2ref)
+        cur["ref2future_lidar_transform"] = np.array(ref2future)
+        cur["total_cur2ref_lidar_transform"] = np.array(cur2ref)
+        cur["total_ref2cur_lidar_transform"] = np.array(ref2cur)
+        metas_all.append(metas)
+        pts_all.append(np.concatenate(pts, 0).astype(np.float32))
+    return dict(img_metas=metas_all, gt_points=pts_all)
